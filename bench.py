@@ -512,6 +512,14 @@ def reference_gpu_leg(dev, maskgit=True):
     return out
 
 
+def dump_outputs(directory, **arrays):
+    """Writes each array as `directory/<name>.npy` in float64 so that two builds can be compared output for output."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), t.detach().cpu().double().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -524,7 +532,11 @@ def main():
     ap.add_argument("--no-refgpu", action="store_true")
     ap.add_argument("--no-train", action="store_true", help="skip the configs[3] training-step block")
     ap.add_argument("--no-makevideo", action="store_true", help="skip the configs[4] make_video block")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the token ids of the last timed encode step to DIR/codebook_ids.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", 0))
     local = int(os.environ.get("LOCAL_RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -589,6 +601,8 @@ def main():
     enc_window = (t_window, time.perf_counter())
     sampler.window = enc_window
     ms_total = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, codebook_ids=ids)
     launches = lib.phk_launch_count() - launches0
     clocks = (sampler.report(enc_window) or None) if rank == 0 else None
     ms_total = S.max_over_ranks(ms_total, dev)   # the job is as slow as its slowest rank
