@@ -351,9 +351,17 @@ int phk_token_embed(const int64_t* ids, const float* tok, const float* pos, floa
  *   l = null + (cond-null)*cond_scale   (null==NULL or cond_scale==1: l = cond)
  *   pred = argmax_v( l/max(T,1e-10) - log(-log(u+1e-10)+1e-10) ), first index on ties
  *   ids = mask ? pred : ids ;  score = mask ? 1 - softmax(l)[pred] : -1e4
- * u: uniform draws [rows, V] (parity mode) or NULL -> in-kernel Philox4x32-10(seed, offset).
+ * u: uniform draws [rows, V] (parity mode) or NULL -> in-kernel noise (seed, offset):
+ *   Philox4x32 with 7 rounds (Random123 definition), key = (seed lo, seed hi), counter =
+ *   (c lo, c hi, 0, 0) with c = offset + r * ceil(V/4) + v/4 (64-bit, wraps mod 2^64) for token
+ *   row r; entry v takes output word v%4.  A row consumes ceil(V/4) counters.
+ *   bits w -> uniform u = (2*(w >> 9) + 1) / 2^24 (exact, strictly inside (0, 1)) ->
+ *   gumbel g = -ln(-ln u), both logarithms in base 2 on the fast-math unit;
+ *   pred = argmax_v( fma(l, 1/max(T,1e-10), g) ), first index on ties.
+ *   phk_noise_probe returns the words and the transform the kernels use.
  * seg_*: token row r reads logits row (r/seg_len)*seg_stride + seg_off + r%seg_len, i.e. the
- * `logits[:, prime_len:]` slice of a primed sample (:503-504); seg_len<=0: identity. */
+ * `logits[:, prime_len:]` slice of a primed sample (:503-504); seg_len<=0: identity.  The noise
+ * counters follow the token row r, not the logits row. */
 int phk_sample_tokens(const float* cond, const float* null_logits, int64_t ld, const float* u,
                       uint64_t seed, uint64_t offset, float cond_scale, float temperature,
                       const uint8_t* mask, int64_t* ids, int64_t* pred_out, float* score_out,
@@ -481,7 +489,8 @@ int phk_layernorm_cfg(const float* x_cond, const float* x_null, const float* gam
  * and reduces argmax / online softmax over the vocabulary straight out of TMEM, so the (b, n, V) logits never exist
  * in memory.  emb bf16 [emb_rows >= n_tokens, dim <= 512] = guided embeddings (phk_layernorm_cfg, or plain norm_out
  * rows when there is no guidance); the 128-token A panel stays resident in shared memory, W streams through TMA.
- * Outputs as phk_sample_tokens. */
+ * Noise as phk_sample_tokens with u == NULL, token t of the call being row r = t: counter offset + t * ceil(V/4) + v/4,
+ * word v%4, the same uniform and gumbel transform.  Outputs as phk_sample_tokens. */
 int64_t phk_head_sample_scratch_bytes(int32_t n_tokens);
 int phk_head_sample(const void* emb, int64_t ld_emb, int64_t emb_rows, const void* W, int64_t ldw, const float* bias,
                     int32_t n_tokens, int32_t V, int32_t dim, float temperature, uint64_t seed, uint64_t offset,
@@ -503,7 +512,8 @@ int phk_head_sample_rng(const void* emb, int64_t ld_emb, int64_t emb_rows, const
  * [b*k, dim] operand, phk_head_sample runs on those rows and the results are scattered back.
  * x_cond / x_null fp32 [b*n, dim]: the residual stream BEFORE norm_out of the two halves; head_w bf16 [V, ldw];
  * mask / ids / pred_out / score_out as phk_sample_tokens, with score = -1e4 and pred = id at unmasked positions;
- * rng_state as phk_head_sample_rng. */
+ * rng_state as phk_head_sample_rng.  The noise counters follow the COMPACT row: the j-th masked position (in position
+ * order) of sequence i draws from counters offset + (i * k + j) * ceil(V/4) + v/4, whatever its position. */
 int64_t phk_sample_tail_scratch_bytes(int32_t b, int32_t k, int32_t dim);
 int phk_sample_tail(const float* x_cond, const float* x_null, const float* gamma, const float* beta, float cond_scale,
                     const void* head_w, int64_t ldw, const float* head_b, int32_t b, int32_t n, int32_t k, int32_t V,
@@ -543,6 +553,12 @@ int phk_maskgit_sample_step_primed(const phk_maskgit_t* m, const int64_t* ids_in
 
 /* rng_state[1] += stride on the stream (device-resident noise key, see phk_head_sample_rng) */
 int phk_rng_advance(uint64_t* rng_state, uint64_t stride, phk_stream_t s);
+
+/* Test hook of the in-kernel sampling noise (phk_sample_tokens with u == NULL): n device entries,
+ * bits_out[i] = Philox word i%4 of counter offset + i/4 under key seed (bits_in == NULL) or bits_in[i];
+ * gumbel_out[i] = the sampling kernels' gumbel transform of that word. */
+int phk_noise_probe(const uint32_t* bits_in, uint64_t seed, uint64_t offset, int64_t n, uint32_t* bits_out,
+                    float* gumbel_out, phk_stream_t s);
 
 /* One WHOLE demasking iteration (phenaki_pytorch.py:485-509, 547-550) as one call:
  *   [k_remask > 0:  mask = scatter(topk(scores, k_remask)); ids = where(mask, mask_id, ids)]      (phk_topk_mask)

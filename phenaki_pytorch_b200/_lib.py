@@ -172,6 +172,7 @@ PROTOTYPES = {
                         i64, vp],
     "phk_head_sample_rng": [vp, i64, i64, vp, i64, vp, i32, i32, i32, f32, u64, u64, vp, vp, vp, vp, vp, vp, i64, vp],
     "phk_rng_advance": [vp, u64, vp],
+    "phk_noise_probe": [vp, u64, u64, i64, vp, vp, vp],
     "phk_debug_step_graph": [i32],
     "phk_vq_cosine_scratch_bytes": [i64, i32, i32],
     "phk_vq_cosine_ids": [vp, vp, vp, vp, i64, i32, i32, vp, i64, i32, vp],

@@ -150,7 +150,11 @@ __device__ __forceinline__ float fast_ex2(float x) {
 // conversion), both logarithms in base 2 on the MUFU unit: g = -ln2 * log2(-log2(u)) - ln(ln 2).
 __device__ __forceinline__ float gumbel_from_bits(uint32_t r) {
   const float u = __uint_as_float(0x3f800000u | (r >> 9)) - 0.99999994f;  // [1, 2) - (1 - 2^-24): exact
-  const float e = -fast_lg2(u);                                           // > 0
+  // e = -log2(u) > 0.  The approximate logarithm's error near 1 (absolute, 2^-22 on [0.5, 2]) is as large as e itself
+  // for the largest u, which decide the argmax; above 1 - 2^-7 e comes from the exact complement w = 1 - u instead:
+  // -ln(1 - w) = w (1 + w/2 + w^2/3 + ...), the two terms kept err by < w^2/3 < 2^-15.5 relative.
+  const float w = 1.0f - u;
+  const float e = u > 0.9921875f ? w * fmaf(w, 0.72134752f, 1.44269504f) : -fast_lg2(u);
   return fmaf(-0.69314718f, fast_lg2(e), 0.36651292f);
 }
 

@@ -128,6 +128,24 @@ __global__ void rng_advance_kernel(unsigned long long* rng_state, unsigned long 
   if (blockIdx.x == 0 && threadIdx.x == 0) rng_state[1] += stride;
 }
 
+// phk_noise_probe: thread q owns counter offset + q, i.e. the four words i = 4q .. 4q+3
+__global__ void noise_probe_kernel(const uint32_t* __restrict__ bits_in, uint64_t seed, uint64_t offset, int64_t n,
+                                   uint32_t* __restrict__ bits_out, float* __restrict__ gumbel_out) {
+  pdl_prologue();
+  for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q * 4 < n; q += (int64_t)gridDim.x * blockDim.x) {
+    uint32_t r[4];
+    if (!bits_in) {
+      const uint64_t ctr = offset + (uint64_t)q;
+      philox4x32<kNoiseRounds>((uint32_t)ctr, (uint32_t)(ctr >> 32), 0u, 0u, (uint32_t)seed, (uint32_t)(seed >> 32), r);
+    }
+    for (int j = 0; j < 4 && q * 4 + j < n; ++j) {
+      const uint32_t w = bits_in ? bits_in[q * 4 + j] : r[j];
+      bits_out[q * 4 + j] = w;
+      gumbel_out[q * 4 + j] = gumbel_from_bits(w);
+    }
+  }
+}
+
 struct TailBufs { int* index; __nv_bfloat16* emb; uint8_t* ones; int64_t* ids_c; int64_t* pred_c; float* score_c; char* head; int64_t head_bytes; };
 
 int64_t align256(int64_t v) { return (v + 255) & ~int64_t(255); }
@@ -215,6 +233,19 @@ extern "C" int phk_rng_advance(uint64_t* rng_state, uint64_t stride, phk_stream_
   PHK_REQUIRE(rng_state, PHK_E_ARG, "phk_rng_advance: null pointer");
   PHK_CUDA(launch_pdl(rng_advance_kernel, dim3(1), dim3(32), (size_t)0, to_stream(s),
                       reinterpret_cast<unsigned long long*>(rng_state), (unsigned long long)stride));
+  PHK_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int phk_noise_probe(const uint32_t* bits_in, uint64_t seed, uint64_t offset, int64_t n, uint32_t* bits_out,
+                               float* gumbel_out, phk_stream_t s) {
+  PHK_REQUIRE(bits_out && gumbel_out, PHK_E_ARG, "phk_noise_probe: null pointer");
+  PHK_REQUIRE(n >= 0, PHK_E_ARG, "phk_noise_probe: bad size");
+  if (n == 0) return 0;
+  const int64_t threads = (n + 3) / 4;
+  const unsigned grid = (unsigned)((threads + 255) / 256 < 4736 ? (threads + 255) / 256 : 4736);
+  PHK_CUDA(launch_pdl(noise_probe_kernel, dim3(grid), dim3(256), (size_t)0, to_stream(s), bits_in, seed, offset, n, bits_out,
+                      gumbel_out));
   PHK_LAUNCH_CHECK();
   return 0;
 }

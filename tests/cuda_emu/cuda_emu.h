@@ -221,7 +221,8 @@ static inline float fast_lg2(float x) { return log2f(x); }
 static inline float fast_ex2(float x) { return exp2f(x); }
 static inline float gumbel_from_bits(uint32_t r) {
   const float u = __uint_as_float(0x3f800000u | (r >> 9)) - 0.99999994f;
-  const float e = -fast_lg2(u);
+  const float w = 1.0f - u;
+  const float e = u > 0.9921875f ? w * fmaf(w, 0.72134752f, 1.44269504f) : -fast_lg2(u);
   return fmaf(-0.69314718f, fast_lg2(e), 0.36651292f);
 }
 
